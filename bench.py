@@ -11,8 +11,8 @@ size on ordinary cudaMalloc buffers:
 
   --impl ours       through the library's public C API (ucc_collective_init / triggered_post / test / finalize), executed by
                     one fused tl/nvl NVLink kernel
-  --impl reference  the reference's own tl/cuda NVLS kernels compiled unmodified from /root/reference and driven through its
-                    stock host sequence (baseline/ref_arm), next to tl/nccl's ncclAllReduce - what its score map falls back to
+  --impl reference  the reference's own tl/cuda NVLS kernels compiled unmodified from an openucx/ucc checkout and driven through
+                    its stock host sequence (oracle/ref_arm), next to tl/nccl's ncclAllReduce - what its score map falls back to
                     for messages above NVLS_SYMMETRIC_SIZE; the better of the two is the reference's value
 
 Device time = CUDA events on the launching stream, max over ranks.  The result vector is verified in full against a
@@ -46,7 +46,16 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-nccl", action="store_true")
     ap.add_argument("--out", default="")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps write what the last timed step of --impl ours computed to DIR/<name>_rank<r>.npy "
+                         "(float32, float64 for --dtype float64; a fixed seeded sample of each vector, at most 32 MB in all): the inputs are "
+                         "the same from run to run, so two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs records the timed path of --impl ours")
+    return a
 
 
 class ClockSampler:
@@ -96,6 +105,25 @@ def pattern(torch, cnt, r, dt, dev, out=None):
         i = torch.arange(o, o + n, device=dev, dtype=torch.int64)
         out[o:o + n] = (((i + 17 * r) % 13) + r).to(dt)
     return out
+
+
+DUMP_BYTES = 16 << 20           # per dumped vector, summed over the ranks
+
+
+def dump_output(torch, d, name, x, rank, N):
+    """DIR/<name>_rank<rank>.npy: the whole of `x` when it fits DUMP_BYTES / N, else its first and last 64 Ki elements plus
+    positions in between drawn from a fixed seed (the same for every run of the same size), in ascending order"""
+    import numpy as np
+    out_dt = torch.float64 if x.dtype == torch.float64 else torch.float32
+    x = x.reshape(-1)
+    k = DUMP_BYTES // (out_dt.itemsize * N)
+    if x.numel() > k:
+        n, edge = x.numel(), min(1 << 16, k // 4)
+        mid = torch.randint(edge, n - edge, (k - 2 * edge,), generator=torch.Generator().manual_seed(20240917))
+        idx = torch.cat([torch.arange(edge), mid, torch.arange(n - edge, n)]).unique()
+        x = x[idx.to(x.device)]
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, f"{name}_rank{rank}.npy"), x.to(out_dt).cpu().numpy())
 
 
 def expected_sum(torch, cnt, N, dt, dev):
@@ -159,9 +187,10 @@ class Bench:
         f = 2.0 * (self.N - 1) / self.N if self.N > 1 else 1.0
         return nbytes / us / 1e3 * f
 
-    def time_arm(self, ar, settle, nbytes, iters, warm, alloc=None):
+    def time_arm(self, ar, settle, nbytes, iters, warm, alloc=None, dump=None):
         """device time per allreduce (us, max over ranks) of `iters` allreduces posted back to back on one stream, and whether
-        the WHOLE result vector of the last one equals the exact expected sum on every rank"""
+        the WHOLE result vector of the last one equals the exact expected sum on every rank; `dump` names the file that result
+        goes to under --dump-outputs"""
         torch = self.torch
         cnt = nbytes // self.esz
         mk = alloc or (lambda c: torch.empty(c, dtype=self.dt, device=self.dev))
@@ -185,6 +214,8 @@ class Bench:
         us = e0.elapsed_time(e1) * 1e3 / iters
         exp = expected_sum(torch, cnt, self.N, self.dt, self.dev)
         ok = bool(torch.equal(dst, exp))
+        if dump and self.a.dump_outputs:
+            dump_output(torch, self.a.dump_outputs, dump, dst, self.rank, self.N)
         del src, dst, exp
         return self.maxr(us), self.all_ok(ok)
 
@@ -234,10 +265,10 @@ def run_ours(a):
             r.wait()                                         # ucc_collective_test + ucc_context_progress
             r.finalize()                                     # ucc_collective_finalize
 
-    def time_ours(nbytes, iters, warm):
+    def time_ours(nbytes, iters, warm, dump=None):
         if use_symm:
             comm.symm_reset()
-        return B.time_arm(ar, settle, nbytes, iters, warm, alloc if use_symm else None)
+        return B.time_arm(ar, settle, nbytes, iters, warm, alloc if use_symm else None, dump)
 
     def time_nccl(nbytes, iters, warm):
         if N == 1 or a.no_nccl:
@@ -259,7 +290,7 @@ def run_ours(a):
     S = a.size
     sampler = ClockSampler(torch.cuda.current_device())
     sampler.start()
-    us, ok = time_ours(S, a.steps, a.warmup)
+    us, ok = time_ours(S, a.steps, a.warmup, dump="allreduce")
     headline_alg = comm.request_info_last()
     value = B.busbw(S, us)
     nccl_us = time_nccl(S, a.steps, a.warmup)
@@ -288,6 +319,8 @@ def run_ours(a):
         e2e_us, last = B.time_e2e(step, S)
         exp = expected_sum(torch, cnt, N, B.dt, B.dev)
         e2e_ok = B.all_ok(bool(torch.equal(dst, exp)))
+        if a.dump_outputs:
+            dump_output(torch, a.dump_outputs, "all_reduce_from_host", dst, B.rank, N)
         e2e = {"value": round(N * B.busbw(S, e2e_us), 3), "busbw_per_gpu_GBps": round(B.busbw(S, e2e_us), 3), "unit": "GB/s", "h2d_bytes_per_step": S,
                "d2h_bytes_per_step": 16 * B.esz, "us_per_step": round(e2e_us, 1), "chunks": ops.last_from_host_chunks(), "correct": e2e_ok,
                "api": "ucc_b200.ops.all_reduce_from_host (pinned host -> device copy pipelined with the tl/nvl allreduce kernels)"}
@@ -316,11 +349,11 @@ def run_ours(a):
 
 # ---------------------------------------------------------------------------------------------------------------------
 def run_reference(a):
-    lib = os.path.join(ROOT, "baseline", "_ref", "libref_tlcuda.so")
+    lib = os.path.join(ROOT, "oracle", "_ref", "libref_tlcuda.so")
     if not os.path.exists(lib):
-        print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref/libref_tlcuda.so is not built (run baseline/ref_arm/build.sh where /root/reference exists)"}))
+        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/libref_tlcuda.so is not built (run oracle/ref_arm/build.sh with REFERENCE_DIR set to an openucx/ucc checkout)"}))
         return 0
-    sys.path.insert(0, os.path.join(ROOT, "baseline", "ref_arm"))
+    sys.path.insert(0, os.path.join(ROOT, "oracle", "ref_arm"))
     B = Bench(a)
     torch, dist, N = B.torch, B.dist, B.N
     S = a.size
@@ -445,7 +478,7 @@ def run_reference(a):
     res["reference_class"] = best
     res["reference_stock_selection"] = stock
     res["reference_arms"] = {k: {"us": round(v[0], 2), "busbw_per_gpu_GBps": round(B.busbw(S, v[0]), 2), "correct": v[1]} for k, v in arms.items()}
-    res["config"]["algorithm"] = "reference openucx/ucc: tl/cuda NVLS kernels (unmodified, baseline/_ref) through the stock memcpy-kernel-memcpy sequence; " \
+    res["config"]["algorithm"] = "reference openucx/ucc: tl/cuda NVLS kernels (unmodified, oracle/_ref) through the stock memcpy-kernel-memcpy sequence; " \
                                  "tl/nccl = ncclAllReduce; value = the faster of the two at the headline size"
     res["gpu_launches_note"] = "launches of the reference's kernels / copies in the timed region (none of the repo's own code is loaded)"
     if tlcuda is not None:

@@ -116,26 +116,34 @@ def test_install_and_consumer_exports(tmp_path):
     assert "CONSUMER_EXPORT_OK" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 
-def test_reference_arm_builds_from_unmodified_reference_sources(tmp_path):
-    """baseline/ref_arm/build.sh: the reference's NVLS kernels are copied byte for byte (sha256 manifests agree) and compile with the two
-    shim headers; bench.py --impl reference then reports through them.  Needs the reference tree and nvcc (skipped elsewhere)."""
-    ref = os.environ.get("REFERENCE_DIR", "/root/reference")
-    if not os.path.isdir(os.path.join(ref, "src", "components", "tl", "cuda", "kernels")) or not os.path.exists("/usr/local/cuda/bin/nvcc"):
-        pytest.skip("reference tree or nvcc not available")
-    env = {k: v for k, v in os.environ.items() if k != "LD_PRELOAD"}   # (tools/run_asan.sh preloads libasan; nvcc does not survive that)
-    r = subprocess.run(["bash", os.path.join(ROOT, "baseline", "ref_arm", "build.sh")], capture_output=True, text=True, timeout=900, env=env)
-    assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-1500:]
-    out = os.path.join(ROOT, "baseline", "_ref")
-    assert os.path.exists(os.path.join(out, "libref_tlcuda.so"))
-    a = sorted(l.split()[0] for l in open(os.path.join(out, "MANIFEST.txt")))
-    b = sorted(l.split()[0] for l in open(os.path.join(out, "MANIFEST.ref.txt")))
-    assert a == b, "a reference source file was altered on its way into baseline/_ref"
+def test_reference_arm_builds_from_unmodified_reference_sources():
+    """oracle/ref_arm/build.sh: the reference's NVLS kernels are copied byte for byte and compile with the two shim headers;
+    bench.py --impl reference then reports through them.  tests/golden/ref_arm_sources.sha256 holds the sha256 of the reference
+    sources the arm was written and measured against: with an openucx/ucc checkout in REFERENCE_DIR the arm is rebuilt from it,
+    and an arm found in oracle/_ref must have been built from exactly those files."""
+    golden = sorted(l for l in open(os.path.join(ROOT, "tests", "golden", "ref_arm_sources.sha256")).read().splitlines() if l)
+    assert len(golden) == 9
+    recipe = open(os.path.join(ROOT, "oracle", "ref_arm", "build.sh")).read()
+    for line in golden:
+        assert os.path.basename(line.split()[1]) in recipe, line
+    # the arm never imports the repository's own package or libraries
+    src = open(os.path.join(ROOT, "oracle", "ref_arm", "ref_arm.py")).read() + open(os.path.join(ROOT, "oracle", "ref_arm", "ref_harness.cpp")).read()
+    assert "ucc_b200" not in src and "libucc" not in src
+    out = os.path.join(ROOT, "oracle", "_ref")
+    ref = os.environ.get("REFERENCE_DIR")
+    if ref and os.path.isdir(os.path.join(ref, "src", "components", "tl", "cuda", "kernels")) and os.path.exists("/usr/local/cuda/bin/nvcc"):
+        env = {k: v for k, v in os.environ.items() if k != "LD_PRELOAD"}   # (tools/run_asan.sh preloads libasan; nvcc does not survive that)
+        r = subprocess.run(["bash", os.path.join(ROOT, "oracle", "ref_arm", "build.sh")], capture_output=True, text=True, timeout=900, env=env)
+        assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-1500:]
+        assert sorted(l for l in open(os.path.join(out, "MANIFEST.ref.txt")).read().splitlines() if l) == golden, \
+            "REFERENCE_DIR is not the reference version the arm was written against"
+    if not os.path.exists(os.path.join(out, "libref_tlcuda.so")):
+        return
+    built = sorted(l for l in open(os.path.join(out, "MANIFEST.txt")).read().splitlines() if l)
+    assert built == golden, "a reference source file was altered on its way into oracle/_ref"
     syms = subprocess.run(["nm", "-D", os.path.join(out, "libref_tlcuda.so")], capture_output=True, text=True).stdout
     for s in ("post_allreduce_kernel", "post_reduce_scatter_kernel", "post_allgatherv_kernel", "ref_allreduce"):
         assert s in syms
-    # the arm never imports the repository's own package or libraries
-    src = open(os.path.join(ROOT, "baseline", "ref_arm", "ref_arm.py")).read() + open(os.path.join(ROOT, "baseline", "ref_arm", "ref_harness.cpp")).read()
-    assert "ucc_b200" not in src and "libucc" not in src
 
 
 def test_bench_pattern_is_exact_in_every_dtype():
@@ -151,3 +159,26 @@ def test_bench_pattern_is_exact_in_every_dtype():
         assert torch.equal(bench.expected_sum(torch, 1000, 8, dt, "cpu").to(torch.float64), exact)
         assert len({float(v) for v in parts[3].to(torch.float64)}) > 5          # not a constant vector
         assert not torch.equal(parts[0], parts[1])
+
+
+def test_bench_dump_output_is_a_fixed_sample(tmp_path):
+    """bench.py --dump-outputs: a large result is sampled at the same positions every run (both ends kept whole) within its byte
+    budget; a small one is written whole; float64 stays float64, every other dtype is written as float32"""
+    torch = pytest.importorskip("torch")
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    x = bench.expected_sum(torch, 2_000_003, 3, torch.bfloat16, "cpu")
+    for d in ("a", "b"):
+        bench.dump_output(torch, str(tmp_path / d), "ar", x, 1, 8)
+    a, b = np.load(tmp_path / "a" / "ar_rank1.npy"), np.load(tmp_path / "b" / "ar_rank1.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, b)
+    assert 0 < a.nbytes <= bench.DUMP_BYTES // 8 and a.size < x.numel()
+    ref = x.float().numpy()
+    assert np.array_equal(a[:1 << 16], ref[:1 << 16]) and np.array_equal(a[-(1 << 16):], ref[-(1 << 16):])
+    y = bench.pattern(torch, 1000, 2, torch.float64, "cpu")
+    bench.dump_output(torch, str(tmp_path / "c"), "small", y, 0, 1)
+    c = np.load(tmp_path / "c" / "small_rank0.npy")
+    assert c.dtype == np.float64 and np.array_equal(c, y.numpy())
