@@ -225,6 +225,18 @@ static int to_nccl_op(ucc_reduction_op_t op, ncclRedOp_t *o)
     switch (op) { case UCC_OP_SUM: *o = ncclSum; break; case UCC_OP_PROD: *o = ncclProd; break; case UCC_OP_MAX: *o = ncclMax; break; case UCC_OP_MIN: *o = ncclMin; break; case UCC_OP_AVG: *o = ncclAvg; break; default: return 0; }
     return 1;
 }
+/* complex SUM / AVG work part by part: NCCL reduces them as a real vector twice as long (as the reference's tl/nccl does);
+ * returns how many real elements one element of udt is, 0 when NCCL cannot reduce (udt, op) */
+static int nccl_red_type(ucc_datatype_t udt, ucc_reduction_op_t uop, ncclDataType_t *dt, ncclRedOp_t *op)
+{
+    if (!to_nccl_op(uop, op)) return 0;
+    if (udt == UCC_DT_FLOAT32_COMPLEX || udt == UCC_DT_FLOAT64_COMPLEX) {
+        if (uop != UCC_OP_SUM && uop != UCC_OP_AVG) return 0;
+        *dt = udt == UCC_DT_FLOAT32_COMPLEX ? ncclFloat32 : ncclFloat64;
+        return 2;
+    }
+    return to_nccl_dt(udt, dt);
+}
 static int cuda_mt(ucc_memory_type_t mt) { return mt == UCC_MEMORY_TYPE_CUDA || mt == UCC_MEMORY_TYPE_CUDA_MANAGED; }
 
 /* the NCCL calls of one collective */
@@ -234,9 +246,9 @@ static ucc_status_t nccl_issue(ucc_tl_nccl_task_t *t, cudaStream_t s)
     ucc_rank_t N = UCC_TL_TEAM_SIZE(team), me = UCC_TL_TEAM_RANK(team); int inplace = UCC_IS_INPLACE(*a), root = (ucc_rank_t)a->root == me;
     ncclDataType_t dt = ncclUint8; ncclRedOp_t op = ncclSum; ncclComm_t c = team->comm;
     switch (a->coll_type) {
-    case UCC_COLL_TYPE_ALLREDUCE:
-        to_nccl_dt(a->dst.info.datatype, &dt); to_nccl_op(a->op, &op);
-        NCCLCHECK(team, nc.AllReduce(inplace ? a->dst.info.buffer : a->src.info.buffer, a->dst.info.buffer, a->dst.info.count, dt, op, c, s)); break;
+    case UCC_COLL_TYPE_ALLREDUCE: {
+        size_t cnt = a->dst.info.count * nccl_red_type(a->dst.info.datatype, a->op, &dt, &op);
+        NCCLCHECK(team, nc.AllReduce(inplace ? a->dst.info.buffer : a->src.info.buffer, a->dst.info.buffer, cnt, dt, op, c, s)); break; }
     case UCC_COLL_TYPE_BARRIER:
         NCCLCHECK(team, nc.AllReduce(NCCL_CTX(team)->barrier_buf, NCCL_CTX(team)->barrier_buf + 1, 1, ncclFloat32, ncclSum, c, s)); break;
     case UCC_COLL_TYPE_ALLGATHER: {
@@ -290,12 +302,12 @@ static ucc_status_t nccl_issue(ucc_tl_nccl_task_t *t, cudaStream_t s)
         } else NCCLCHECK(team, nc.Broadcast(a->src.info.buffer, a->src.info.buffer, a->src.info.count * ucc_dt_size(a->src.info.datatype), ncclUint8, (int)a->root, c, s));
         break;
     case UCC_COLL_TYPE_REDUCE_SCATTER: {
-        size_t cnt = inplace ? a->dst.info.count / N : a->dst.info.count;
-        to_nccl_dt(a->dst.info.datatype, &dt); to_nccl_op(a->op, &op);
-        NCCLCHECK(team, nc.ReduceScatter(inplace ? a->dst.info.buffer : a->src.info.buffer, inplace ? (char *)a->dst.info.buffer + me * cnt * ucc_dt_size(a->dst.info.datatype) : a->dst.info.buffer, cnt, dt, op, c, s)); break; }
+        size_t cnt = inplace ? a->dst.info.count / N : a->dst.info.count, mine = me * cnt * ucc_dt_size(a->dst.info.datatype);
+        cnt *= nccl_red_type(a->dst.info.datatype, a->op, &dt, &op);
+        NCCLCHECK(team, nc.ReduceScatter(inplace ? a->dst.info.buffer : a->src.info.buffer, inplace ? (char *)a->dst.info.buffer + mine : a->dst.info.buffer, cnt, dt, op, c, s)); break; }
     case UCC_COLL_TYPE_REDUCE: {
         ucc_datatype_t udt = root ? a->dst.info.datatype : a->src.info.datatype; size_t cnt = root ? a->dst.info.count : a->src.info.count;
-        to_nccl_dt(udt, &dt); to_nccl_op(a->op, &op);
+        cnt *= nccl_red_type(udt, a->op, &dt, &op);
         NCCLCHECK(team, nc.Reduce((root && inplace) ? a->dst.info.buffer : a->src.info.buffer, root ? a->dst.info.buffer : NULL, cnt, dt, op, (int)a->root, c, s)); break; }
     case UCC_COLL_TYPE_GATHER: case UCC_COLL_TYPE_GATHERV: {
         int v = a->coll_type == UCC_COLL_TYPE_GATHERV;
@@ -378,7 +390,7 @@ static ucc_status_t nccl_coll_init_alg(ucc_base_coll_args_t *b, ucc_base_team_t 
     if (ucc_coll_has_reduction(a->coll_type)) {
         int root = (ucc_rank_t)a->root == UCC_TL_TEAM_RANK(team);
         ucc_datatype_t udt = (a->coll_type == UCC_COLL_TYPE_REDUCE && !root) ? a->src.info.datatype : a->dst.info.datatype;
-        if (!to_nccl_dt(udt, &dt) || !to_nccl_op(a->op, &op)) return UCC_ERR_NOT_SUPPORTED;
+        if (!nccl_red_type(udt, a->op, &dt, &op)) return UCC_ERR_NOT_SUPPORTED;
     }
     if ((a->coll_type & (UCC_COLL_TYPE_ALLTOALL | UCC_COLL_TYPE_ALLTOALLV)) && UCC_IS_INPLACE(*a)) return UCC_ERR_NOT_SUPPORTED;
     if (UCC_COLL_ARGS_ACTIVE_SET(a) && a->coll_type != UCC_COLL_TYPE_BCAST) return UCC_ERR_NOT_SUPPORTED;

@@ -156,6 +156,14 @@ template <typename T> NVL_DEV void store_dst_vec(T *base, size_t idx, size_t n, 
 /* ------------------------------------------------------------------ */
 /* reduction templates                                                 */
 /* ------------------------------------------------------------------ */
+/* complex elements (UCC_DT_FLOAT32_COMPLEX / FLOAT64_COMPLEX): plain pairs aligned like their component (4 / 8 bytes, not 16),
+ * so the guarded element path (base[idx + i]) never issues an access wider than the alignment the caller's buffer has */
+struct nvl_c64 { float re, im; };
+struct nvl_c128 { double re, im; };
+template <typename T> struct IsComplex { static constexpr bool v = false; };
+template <> struct IsComplex<nvl_c64> { static constexpr bool v = true; };
+template <> struct IsComplex<nvl_c128> { static constexpr bool v = true; };
+
 template <typename T> struct AccOf { typedef T type; };
 template <> struct AccOf<__half> { typedef float type; };
 template <> struct AccOf<__nv_bfloat16> { typedef float type; };
@@ -179,6 +187,16 @@ template <typename A> struct OpFn<NVL_OP_LXOR, A> { static NVL_DEV A f(A a, A b)
 template <typename A> struct OpFn<NVL_OP_BAND, A> { static NVL_DEV A f(A a, A b) { return (A)(a & b); } };
 template <typename A> struct OpFn<NVL_OP_BOR, A> { static NVL_DEV A f(A a, A b) { return (A)(a | b); } };
 template <typename A> struct OpFn<NVL_OP_BXOR, A> { static NVL_DEV A f(A a, A b) { return (A)(a ^ b); } };
+/* complex: SUM / AVG part by part, PROD = (ac - bd) + (ad + bc)i as cuCmul computes it (no Annex G inf / nan recovery);
+ * accumulation stays in the component precision */
+#define NVL_COMPLEX_OPS(_C)                                                                                                  \
+    template <> struct OpFn<NVL_OP_SUM, _C> { static NVL_DEV _C f(_C a, _C b) { return {a.re + b.re, a.im + b.im}; } };     \
+    template <> struct OpFn<NVL_OP_AVG, _C> { static NVL_DEV _C f(_C a, _C b) { return {a.re + b.re, a.im + b.im}; } };     \
+    template <> struct OpFn<NVL_OP_PROD, _C> {                                                                              \
+        static NVL_DEV _C f(_C a, _C b) { return {a.re * b.re - a.im * b.im, a.re * b.im + a.im * b.re}; } };
+NVL_COMPLEX_OPS(nvl_c64)
+NVL_COMPLEX_OPS(nvl_c128)
+#undef NVL_COMPLEX_OPS
 
 /* AVG = SUM scaled by 1/N at the very end.  Floating types multiply by 1/N; integer types divide by N (truncating, i.e. what
  * the reference's d[i] * (1/N) in double precision yields for every sum a double represents exactly) - casting 1/N to an integer
@@ -189,7 +207,8 @@ template <> struct IsIntAcc<double> { static constexpr bool v = false; };
 template <int OP, typename A> NVL_DEV A avg_scale(A x, float inv_n, int n)
 {
     if (OP != NVL_OP_AVG) return x;
-    if constexpr (IsIntAcc<A>::v) return n > 1 ? (A)(x / (A)n) : x;
+    if constexpr (IsComplex<A>::v) { typedef decltype(x.re) R; const R s = (R)1 / (R)n; return {x.re * s, x.im * s}; } /* 1/N in the component precision (IsIntAcc is true for it) */
+    else if constexpr (IsIntAcc<A>::v) return n > 1 ? (A)(x / (A)n) : x;
     else return (A)(x * (A)inv_n);
 }
 
@@ -216,25 +235,32 @@ template <> struct IsFloatLike<double> { static constexpr bool v = true; };
 template <> struct IsFloatLike<__half> { static constexpr bool v = true; };
 template <> struct IsFloatLike<__nv_bfloat16> { static constexpr bool v = true; };
 
-/* run F<T,OP>::run(args...) for the runtime operator; bit/logic operators only exist for integer types */
+/* run F<T,OP>::run(args...) for the runtime operator; MAX / MIN do not exist for complex types, bit/logic operators only for
+ * integer types */
 #define NVL_DISPATCH_OP(_T, _op, _CALL)                                                         \
     do {                                                                                        \
         switch (_op) {                                                                          \
         case NVL_OP_SUM: _CALL(_T, NVL_OP_SUM); break;                                          \
         case NVL_OP_AVG: _CALL(_T, NVL_OP_AVG); break;                                          \
         case NVL_OP_PROD: _CALL(_T, NVL_OP_PROD); break;                                        \
-        case NVL_OP_MAX: _CALL(_T, NVL_OP_MAX); break;                                          \
-        case NVL_OP_MIN: _CALL(_T, NVL_OP_MIN); break;                                          \
         default:                                                                                \
-            if constexpr (!IsFloatLike<_T>::v) {                                                \
+            if constexpr (!IsComplex<_T>::v) {                                                  \
                 switch (_op) {                                                                  \
-                case NVL_OP_LAND: _CALL(_T, NVL_OP_LAND); break;                                \
-                case NVL_OP_LOR: _CALL(_T, NVL_OP_LOR); break;                                  \
-                case NVL_OP_LXOR: _CALL(_T, NVL_OP_LXOR); break;                                \
-                case NVL_OP_BAND: _CALL(_T, NVL_OP_BAND); break;                                \
-                case NVL_OP_BOR: _CALL(_T, NVL_OP_BOR); break;                                  \
-                case NVL_OP_BXOR: _CALL(_T, NVL_OP_BXOR); break;                                \
-                default: break;                                                                 \
+                case NVL_OP_MAX: _CALL(_T, NVL_OP_MAX); break;                                  \
+                case NVL_OP_MIN: _CALL(_T, NVL_OP_MIN); break;                                  \
+                default:                                                                        \
+                    if constexpr (!IsFloatLike<_T>::v) {                                        \
+                        switch (_op) {                                                          \
+                        case NVL_OP_LAND: _CALL(_T, NVL_OP_LAND); break;                        \
+                        case NVL_OP_LOR: _CALL(_T, NVL_OP_LOR); break;                          \
+                        case NVL_OP_LXOR: _CALL(_T, NVL_OP_LXOR); break;                        \
+                        case NVL_OP_BAND: _CALL(_T, NVL_OP_BAND); break;                        \
+                        case NVL_OP_BOR: _CALL(_T, NVL_OP_BOR); break;                          \
+                        case NVL_OP_BXOR: _CALL(_T, NVL_OP_BXOR); break;                        \
+                        default: break;                                                         \
+                        }                                                                       \
+                    }                                                                           \
+                    break;                                                                      \
                 }                                                                               \
             }                                                                                   \
             break;                                                                              \

@@ -214,7 +214,7 @@ __global__ void __launch_bounds__(NVL_THREADS_MAX, 2) nvl_exchange_kernel(nvl_xc
 #ifndef NVL_HOST_EMU /* tests/emu includes the kernels above and calls them directly */
 extern "C" size_t nvl_dt_size(int dt)
 {
-    static const size_t s[NVL_DT_LAST] = {1, 2, 4, 8, 1, 2, 4, 8, 2, 4, 8, 2};
+    static const size_t s[NVL_DT_LAST] = {1, 2, 4, 8, 1, 2, 4, 8, 2, 4, 8, 2, 8, 16};
     return dt >= 0 && dt < NVL_DT_LAST ? s[dt] : 0;
 }
 extern "C" int nvl_dt_supports_op(int dt, int op)
@@ -222,12 +222,13 @@ extern "C" int nvl_dt_supports_op(int dt, int op)
     if (dt < 0 || dt >= NVL_DT_LAST || op < 0 || op >= NVL_OP_LAST) return 0;
     if (dt == NVL_DT_F16 || dt == NVL_DT_F32 || dt == NVL_DT_F64 || dt == NVL_DT_BF16)
         return op == NVL_OP_SUM || op == NVL_OP_PROD || op == NVL_OP_MAX || op == NVL_OP_MIN || op == NVL_OP_AVG;
+    if (dt == NVL_DT_C64 || dt == NVL_DT_C128) return op == NVL_OP_SUM || op == NVL_OP_PROD || op == NVL_OP_AVG;
     return 1;
 }
 extern "C" int nvl_nvls_supports(int dt, int op)
 {
     /* mirrors the McRed<T,OP> specialisations: what multimem.ld_reduce can do for 16-byte vectors of that type */
-    if (dt == NVL_DT_F32 || dt == NVL_DT_BF16 || dt == NVL_DT_F16) return op == NVL_OP_SUM || op == NVL_OP_AVG;
+    if (dt == NVL_DT_F32 || dt == NVL_DT_BF16 || dt == NVL_DT_F16 || dt == NVL_DT_C64) return op == NVL_OP_SUM || op == NVL_OP_AVG;
     if (dt == NVL_DT_I32 || dt == NVL_DT_U32 || dt == NVL_DT_I64 || dt == NVL_DT_U64)
         return op == NVL_OP_SUM || op == NVL_OP_MIN || op == NVL_OP_MAX || op == NVL_OP_BAND || op == NVL_OP_BOR || op == NVL_OP_BXOR;
     return 0;
@@ -236,11 +237,13 @@ extern "C" int nvl_nvls_supports(int dt, int op)
 typedef cudaError_t (*nvl_red_launch_fn)(const nvl_red_args_t *, int, int, cudaStream_t);
 #define DECL(_s) extern "C" cudaError_t nvl_launch_oneshot_##_s(const nvl_red_args_t *, int, int, cudaStream_t); \
                  extern "C" cudaError_t nvl_launch_staged_##_s(const nvl_red_args_t *, int, int, cudaStream_t);
-DECL(i8) DECL(i16) DECL(i32) DECL(i64) DECL(u8) DECL(u16) DECL(u32) DECL(u64) DECL(f16) DECL(f32) DECL(f64) DECL(bf16)
+DECL(i8) DECL(i16) DECL(i32) DECL(i64) DECL(u8) DECL(u16) DECL(u32) DECL(u64) DECL(f16) DECL(f32) DECL(f64) DECL(bf16) DECL(c64) DECL(c128)
 static const nvl_red_launch_fn oneshot_fns[NVL_DT_LAST] = {nvl_launch_oneshot_i8, nvl_launch_oneshot_i16, nvl_launch_oneshot_i32, nvl_launch_oneshot_i64, nvl_launch_oneshot_u8, nvl_launch_oneshot_u16,
-    nvl_launch_oneshot_u32, nvl_launch_oneshot_u64, nvl_launch_oneshot_f16, nvl_launch_oneshot_f32, nvl_launch_oneshot_f64, nvl_launch_oneshot_bf16};
+    nvl_launch_oneshot_u32, nvl_launch_oneshot_u64, nvl_launch_oneshot_f16, nvl_launch_oneshot_f32, nvl_launch_oneshot_f64, nvl_launch_oneshot_bf16,
+    nvl_launch_oneshot_c64, nvl_launch_oneshot_c128};
 static const nvl_red_launch_fn staged_fns[NVL_DT_LAST] = {nvl_launch_staged_i8, nvl_launch_staged_i16, nvl_launch_staged_i32, nvl_launch_staged_i64, nvl_launch_staged_u8, nvl_launch_staged_u16,
-    nvl_launch_staged_u32, nvl_launch_staged_u64, nvl_launch_staged_f16, nvl_launch_staged_f32, nvl_launch_staged_f64, nvl_launch_staged_bf16};
+    nvl_launch_staged_u32, nvl_launch_staged_u64, nvl_launch_staged_f16, nvl_launch_staged_f32, nvl_launch_staged_f64, nvl_launch_staged_bf16,
+    nvl_launch_staged_c64, nvl_launch_staged_c128};
 
 extern "C" cudaError_t nvl_launch_allreduce_oneshot(const nvl_red_args_t *a, int nblocks, int nthreads, cudaStream_t s)
 {
@@ -255,9 +258,10 @@ extern "C" cudaError_t nvl_launch_reduce_staged(const nvl_red_args_t *a, int nbl
     return staged_fns[a->dt](a, nblocks, nthreads, s);
 }
 #define DECLD(_s) extern "C" cudaError_t nvl_launch_direct_##_s(const nvl_red_args_t *, int, int, cudaStream_t);
-DECLD(i8) DECLD(i16) DECLD(i32) DECLD(i64) DECLD(u8) DECLD(u16) DECLD(u32) DECLD(u64) DECLD(f16) DECLD(f32) DECLD(f64) DECLD(bf16)
+DECLD(i8) DECLD(i16) DECLD(i32) DECLD(i64) DECLD(u8) DECLD(u16) DECLD(u32) DECLD(u64) DECLD(f16) DECLD(f32) DECLD(f64) DECLD(bf16) DECLD(c64) DECLD(c128)
 static const nvl_red_launch_fn direct_fns[NVL_DT_LAST] = {nvl_launch_direct_i8, nvl_launch_direct_i16, nvl_launch_direct_i32, nvl_launch_direct_i64, nvl_launch_direct_u8, nvl_launch_direct_u16,
-    nvl_launch_direct_u32, nvl_launch_direct_u64, nvl_launch_direct_f16, nvl_launch_direct_f32, nvl_launch_direct_f64, nvl_launch_direct_bf16};
+    nvl_launch_direct_u32, nvl_launch_direct_u64, nvl_launch_direct_f16, nvl_launch_direct_f32, nvl_launch_direct_f64, nvl_launch_direct_bf16,
+    nvl_launch_direct_c64, nvl_launch_direct_c128};
 extern "C" cudaError_t nvl_launch_reduce_direct(const nvl_red_args_t *a, int nblocks, int nthreads, cudaStream_t s)
 {
     if (nthreads > NVL_THREADS_MAX) nthreads = NVL_THREADS_MAX;
@@ -265,9 +269,10 @@ extern "C" cudaError_t nvl_launch_reduce_direct(const nvl_red_args_t *a, int nbl
     return direct_fns[a->dt](a, nblocks, nthreads, s);
 }
 #define DECLS(_s) extern "C" cudaError_t nvl_launch_steps_##_s(const nvl_red_args_t *, int, int, cudaStream_t);
-DECLS(i8) DECLS(i16) DECLS(i32) DECLS(i64) DECLS(u8) DECLS(u16) DECLS(u32) DECLS(u64) DECLS(f16) DECLS(f32) DECLS(f64) DECLS(bf16)
+DECLS(i8) DECLS(i16) DECLS(i32) DECLS(i64) DECLS(u8) DECLS(u16) DECLS(u32) DECLS(u64) DECLS(f16) DECLS(f32) DECLS(f64) DECLS(bf16) DECLS(c64) DECLS(c128)
 static const nvl_red_launch_fn steps_fns[NVL_DT_LAST] = {nvl_launch_steps_i8, nvl_launch_steps_i16, nvl_launch_steps_i32, nvl_launch_steps_i64, nvl_launch_steps_u8, nvl_launch_steps_u16,
-    nvl_launch_steps_u32, nvl_launch_steps_u64, nvl_launch_steps_f16, nvl_launch_steps_f32, nvl_launch_steps_f64, nvl_launch_steps_bf16};
+    nvl_launch_steps_u32, nvl_launch_steps_u64, nvl_launch_steps_f16, nvl_launch_steps_f32, nvl_launch_steps_f64, nvl_launch_steps_bf16,
+    nvl_launch_steps_c64, nvl_launch_steps_c128};
 extern "C" cudaError_t nvl_launch_reduce_steps(const nvl_red_args_t *a, int nblocks, int nthreads, cudaStream_t s)
 {
     if (nthreads > NVL_THREADS_MAX) nthreads = NVL_THREADS_MAX;

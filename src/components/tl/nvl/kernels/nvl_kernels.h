@@ -60,7 +60,7 @@ typedef struct nvl_team_dev {
 } nvl_team_dev_t;
 
 typedef enum { NVL_DT_I8, NVL_DT_I16, NVL_DT_I32, NVL_DT_I64, NVL_DT_U8, NVL_DT_U16, NVL_DT_U32, NVL_DT_U64,
-               NVL_DT_F16, NVL_DT_F32, NVL_DT_F64, NVL_DT_BF16, NVL_DT_LAST } nvl_dt_t;
+               NVL_DT_F16, NVL_DT_F32, NVL_DT_F64, NVL_DT_BF16, NVL_DT_C64, NVL_DT_C128, NVL_DT_LAST } nvl_dt_t;
 typedef enum { NVL_OP_SUM, NVL_OP_PROD, NVL_OP_MAX, NVL_OP_MIN, NVL_OP_LAND, NVL_OP_LOR, NVL_OP_LXOR, NVL_OP_BAND, NVL_OP_BOR,
                NVL_OP_BXOR, NVL_OP_AVG, NVL_OP_LAST } nvl_op_t;
 

@@ -86,6 +86,8 @@ extern "C" cudaError_t nvl_launch_reduce_scatter_oneshot(const nvl_red_args_t *a
     case NVL_DT_F32: return nvl_reduce_scatter_oneshot_kernel_launch<float>(a, nblocks, nthreads, s);
     case NVL_DT_F64: return nvl_reduce_scatter_oneshot_kernel_launch<double>(a, nblocks, nthreads, s);
     case NVL_DT_BF16: return nvl_reduce_scatter_oneshot_kernel_launch<__nv_bfloat16>(a, nblocks, nthreads, s);
+    case NVL_DT_C64: return nvl_reduce_scatter_oneshot_kernel_launch<nvl_c64>(a, nblocks, nthreads, s);
+    case NVL_DT_C128: return nvl_reduce_scatter_oneshot_kernel_launch<nvl_c128>(a, nblocks, nthreads, s);
     default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();

@@ -146,6 +146,8 @@ template <typename T, int OP> struct McRed { static __device__ __forceinline__ u
 NVL_MCRED(float, NVL_OP_SUM, mc_ld_reduce_f32) NVL_MCRED(float, NVL_OP_AVG, mc_ld_reduce_f32)
 NVL_MCRED(__half, NVL_OP_SUM, mc_ld_reduce_f16) NVL_MCRED(__half, NVL_OP_AVG, mc_ld_reduce_f16)
 NVL_MCRED(__nv_bfloat16, NVL_OP_SUM, mc_ld_reduce_bf16) NVL_MCRED(__nv_bfloat16, NVL_OP_AVG, mc_ld_reduce_bf16)
+/* c64 SUM / AVG are f32 adds part by part; c128 would need the scalar f64 form, which would also move f64 onto this path */
+NVL_MCRED(nvl_c64, NVL_OP_SUM, mc_ld_reduce_f32) NVL_MCRED(nvl_c64, NVL_OP_AVG, mc_ld_reduce_f32)
 NVL_MCRED(int32_t, NVL_OP_SUM, mc_red_add_s32) NVL_MCRED(int32_t, NVL_OP_MIN, mc_red_min_s32) NVL_MCRED(int32_t, NVL_OP_MAX, mc_red_max_s32)
 NVL_MCRED(int32_t, NVL_OP_BAND, mc_red_and_b32) NVL_MCRED(int32_t, NVL_OP_BOR, mc_red_or_b32) NVL_MCRED(int32_t, NVL_OP_BXOR, mc_red_xor_b32)
 NVL_MCRED(uint32_t, NVL_OP_SUM, mc_red_add_u32) NVL_MCRED(uint32_t, NVL_OP_MIN, mc_red_min_u32) NVL_MCRED(uint32_t, NVL_OP_MAX, mc_red_max_u32)

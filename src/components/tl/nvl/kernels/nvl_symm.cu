@@ -110,6 +110,7 @@ extern "C" cudaError_t nvl_launch_reduce_symm(const nvl_red_args_t *a, int nbloc
     case NVL_DT_U32: return nvl_allreduce_symm_kernel_launch<uint32_t>(a, nblocks, nthreads, s);
     case NVL_DT_I64: return nvl_allreduce_symm_kernel_launch<int64_t>(a, nblocks, nthreads, s);
     case NVL_DT_U64: return nvl_allreduce_symm_kernel_launch<uint64_t>(a, nblocks, nthreads, s);
+    case NVL_DT_C64: return nvl_allreduce_symm_kernel_launch<nvl_c64>(a, nblocks, nthreads, s);
     default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();

@@ -17,6 +17,7 @@ static int to_nvl_dt(ucc_datatype_t dt)
     case UCC_DT_INT8: return NVL_DT_I8; case UCC_DT_INT16: return NVL_DT_I16; case UCC_DT_INT32: return NVL_DT_I32; case UCC_DT_INT64: return NVL_DT_I64;
     case UCC_DT_UINT8: return NVL_DT_U8; case UCC_DT_UINT16: return NVL_DT_U16; case UCC_DT_UINT32: return NVL_DT_U32; case UCC_DT_UINT64: return NVL_DT_U64;
     case UCC_DT_FLOAT16: return NVL_DT_F16; case UCC_DT_FLOAT32: return NVL_DT_F32; case UCC_DT_FLOAT64: return NVL_DT_F64; case UCC_DT_BFLOAT16: return NVL_DT_BF16;
+    case UCC_DT_FLOAT32_COMPLEX: return NVL_DT_C64; case UCC_DT_FLOAT64_COMPLEX: return NVL_DT_C128;
     default: return -1;
     }
 }

@@ -35,9 +35,10 @@ ROOTED = {"bcast", "reduce", "gather", "gatherv", "scatter", "scatterv"}
 NO_DATA = {"barrier"}
 NP_DT = {"int8": np.int8, "uint8": np.uint8, "int16": np.int16, "uint16": np.uint16, "int32": np.int32, "uint32": np.uint32,
          "int64": np.int64, "uint64": np.uint64, "float16": np.float16, "float32": np.float32, "float64": np.float64,
-         "bfloat16": None}
+         "bfloat16": None, "float32_complex": np.complex64, "float64_complex": np.complex128}
 INT_OPS = {"sum", "prod", "max", "min", "land", "lor", "lxor", "band", "bor", "bxor"}
 FLOAT_OPS = {"sum", "prod", "max", "min", "avg"}
+COMPLEX_OPS = {"sum", "prod", "avg"}   # what the reference's ec/cuda defines for complex types
 MEM = {"host": U.UCC_MEMORY_TYPE_HOST, "cuda": U.UCC_MEMORY_TYPE_CUDA, "cudaManaged": U.UCC_MEMORY_TYPE_CUDA_MANAGED}
 
 
@@ -46,7 +47,16 @@ def dt_size(dt):
 
 
 def is_float(dt):
-    return dt in ("float16", "float32", "float64", "bfloat16")
+    return dt in ("float16", "float32", "float64", "bfloat16", "float32_complex", "float64_complex")
+
+
+def is_complex(dt):
+    return dt in ("float32_complex", "float64_complex")
+
+
+def logical_dt(dt):
+    """numpy type the logical contents of a `dt` buffer travel in"""
+    return np.complex128 if is_complex(dt) else np.float64 if is_float(dt) else np.int64
 
 
 class Buf:
@@ -84,12 +94,18 @@ class Buf:
         if self.dt == "bfloat16":
             return raw.view(torch.bfloat16).float().numpy().astype(np.float64)
         v = raw.numpy().view(NP_DT[self.dt])
-        return v.astype(np.float64 if is_float(self.dt) else (np.uint64 if self.dt == "uint64" else np.int64))
+        return v.astype(np.uint64 if self.dt == "uint64" else logical_dt(self.dt))
 
 
 def gen(seed, case, rank, count, dt, op="sum"):
     """logical input of `rank`: small non-negative values, exactly representable in every datatype"""
     g = np.random.default_rng([seed, case, rank])
+    if is_complex(dt):   # Gaussian integers: sums exact; PROD parts in [-1, 1] (never 0) keep products of many ranks small
+        lo, hi = (-1, 2) if op == "prod" else (-4, 5)
+        re, im = g.integers(lo, hi, count), g.integers(lo, hi, count)
+        if op == "prod":
+            re[(re == 0) & (im == 0)] = 1
+        return (re + 1j * im).astype(np.complex128)
     if op == "prod":
         return g.integers(1, 3, count).astype(np.float64 if is_float(dt) else np.int64)
     hi = 4 if dt in ("int8", "uint8", "float16", "bfloat16") else 100
@@ -100,6 +116,9 @@ def reduce_oracle(op, arrs, dt):
     a = np.stack(arrs)
     if op == "sum":
         r = a.sum(0)
+    elif op == "avg" and is_complex(dt):   # the sum times 1/N computed in the component precision
+        c = NP_DT[dt](0).real.dtype.type
+        r = (a.sum(0).astype(NP_DT[dt]) * (c(1) / c(len(arrs)))).astype(np.complex128)
     elif op == "avg":
         r = a.sum(0) / len(arrs)
     elif op == "prod":
@@ -125,7 +144,10 @@ def reduce_oracle(op, arrs, dt):
 def close(got, exp, dt, n):
     if not is_float(dt):
         return np.array_equal(got.astype(np.int64), np.asarray(exp).astype(np.int64))
-    tol = {"float64": 1e-12, "float32": 1e-5, "float16": 2e-2, "bfloat16": 6e-2}[dt] * max(1, n)
+    tol = {"float64": 1e-12, "float32": 1e-5, "float16": 2e-2, "bfloat16": 6e-2, "float64_complex": 1e-12, "float32_complex": 1e-5}[dt] * max(1, n)
+    if is_complex(dt):   # per part, with the tolerance of the component type
+        exp = np.asarray(exp)
+        return np.allclose(got.real, exp.real, rtol=tol, atol=tol) and np.allclose(got.imag, exp.imag, rtol=tol, atol=tol)
     return np.allclose(got, exp, rtol=tol, atol=tol)
 
 
@@ -232,7 +254,7 @@ def build_case(coll, team, urank, n, seed, case, dt, op, mtype, count, root, inp
         exp = np.concatenate(data) if sum(counts) else np.zeros(0)
         dst = buf(sum(counts))
         if inplace:
-            full = np.zeros(sum(counts), np.float64 if is_float(dt) else np.int64)
+            full = np.zeros(sum(counts), logical_dt(dt))
             full[displs[urank]:displs[urank] + counts[urank]] = data[urank]
             dst.set(full)
             a = coll_args(coll, dt=dt, inplace=True, mem_type=mt, dst_ptr=dst.ptr, dst_counts=counts, dst_displs=displs, count_src=0)
@@ -296,7 +318,7 @@ def build_case(coll, team, urank, n, seed, case, dt, op, mtype, count, root, inp
         src = buf(counts[urank], data[urank])
         dst = buf(sum(counts)) if is_root else None
         if inplace and is_root:
-            full = np.zeros(sum(counts), np.float64 if is_float(dt) else np.int64)
+            full = np.zeros(sum(counts), logical_dt(dt))
             full[displs[urank]:displs[urank] + counts[urank]] = data[urank]
             dst.set(full)
             if coll == "gather":
@@ -478,7 +500,7 @@ def main(argv=None):
                 case += 1
                 if dt not in NP_DT or mtype not in MEM:
                     raise SystemExit(f"incorrect dtype/mtype: {dt}/{mtype}")
-                if coll in REDUCTIONS and op not in (FLOAT_OPS if is_float(dt) else INT_OPS):
+                if coll in REDUCTIONS and op not in (COMPLEX_OPS if is_complex(dt) else FLOAT_OPS if is_float(dt) else INT_OPS):
                     continue
                 if trig and mtype != "cuda":
                     continue
