@@ -56,7 +56,7 @@ template <typename T, int OP> static __device__ __forceinline__ void reduce_body
 #pragma unroll
             for (int i = 0; i < E; i++) acc.a[i] = scale<A>(acc.a[i], a.alpha);
         }
-        st_v4((char *)a.dst + v * 16, acc.get(1.0f, 1));
+        st_v4((char *)a.dst + v * 16, acc.get(1));
     }
     reduce_scalar<T, A, OP>(a, nvec * E, a.count, [](T x) { return to_acc<T>(x); }, [](A x) { return from_acc<T>(x); }, tid, nt);
 }

@@ -198,18 +198,19 @@ NVL_COMPLEX_OPS(nvl_c64)
 NVL_COMPLEX_OPS(nvl_c128)
 #undef NVL_COMPLEX_OPS
 
-/* AVG = SUM scaled by 1/N at the very end.  Floating types multiply by 1/N; integer types divide by N (truncating, i.e. what
- * the reference's d[i] * (1/N) in double precision yields for every sum a double represents exactly) - casting 1/N to an integer
- * accumulator would be 0 */
+/* AVG = SUM scaled by 1/N at the very end.  Floating types multiply by 1/N computed in the accumulator's precision (float for
+ * f16 / bf16 / f32, double for f64; a float 1/N would cost f64 about 1e-8 relative for N = 3); integer types divide by N
+ * (truncating, i.e. what the reference's d[i] * (1/N) in double precision yields for every sum a double represents exactly) -
+ * casting 1/N to an integer accumulator would be 0 */
 template <typename A> struct IsIntAcc { static constexpr bool v = true; };
 template <> struct IsIntAcc<float> { static constexpr bool v = false; };
 template <> struct IsIntAcc<double> { static constexpr bool v = false; };
-template <int OP, typename A> NVL_DEV A avg_scale(A x, float inv_n, int n)
+template <int OP, typename A> NVL_DEV A avg_scale(A x, int n)
 {
     if (OP != NVL_OP_AVG) return x;
     if constexpr (IsComplex<A>::v) { typedef decltype(x.re) R; const R s = (R)1 / (R)n; return {x.re * s, x.im * s}; } /* 1/N in the component precision (IsIntAcc is true for it) */
     else if constexpr (IsIntAcc<A>::v) return n > 1 ? (A)(x / (A)n) : x;
-    else return (A)(x * (A)inv_n);
+    else return (A)(x * ((A)1 / (A)n));
 }
 
 /* accumulator for one 16-byte vector of T */
@@ -223,9 +224,9 @@ template <typename T, int OP> struct VecAcc {
     NVL_DEV void add(uint4 x) { Vec<T> u; u.v = x;
 #pragma unroll
         for (int i = 0; i < E; i++) a[i] = OpFn<OP, A>::f(a[i], to_acc<T>(u.e[i])); }
-    NVL_DEV uint4 get(float inv_n, int n) { Vec<T> u;
+    NVL_DEV uint4 get(int n) { Vec<T> u;
 #pragma unroll
-        for (int i = 0; i < E; i++) u.e[i] = from_acc<T>(avg_scale<OP, A>(a[i], inv_n, n));
+        for (int i = 0; i < E; i++) u.e[i] = from_acc<T>(avg_scale<OP, A>(a[i], n));
         return u.v; }
 };
 

@@ -45,10 +45,19 @@ template <typename E, typename F> static inline uint4 emu_mc_reduce(const void *
     uint4 v; memcpy(&v, acc, 16); return v;
 }
 static inline uint4 mc_ld_reduce_f32(const void *mc) { return emu_mc_reduce<float>(mc, [](float a, float b) { return a + b; }); }
+/* .acc::f32: the switch adds the 16-bit values in float and rounds the sum once to the storage type */
+template <typename H, typename TO, typename FROM> static inline uint4 emu_mc_reduce_acc_f32(const void *mc, TO to_f, FROM from_f)
+{
+    const size_t off = emu_mc_off(mc);
+    H cur[8]; float acc[8];
+    for (int p = 0; p < g_emu.n; p++) { memcpy(cur, g_emu.heaps[p] + off, 16); for (int i = 0; i < 8; i++) acc[i] = p ? acc[i] + to_f(cur[i]) : to_f(cur[i]); }
+    for (int i = 0; i < 8; i++) cur[i] = from_f(acc[i]);
+    uint4 v; memcpy(&v, cur, 16); return v;
+}
 static inline uint4 mc_ld_reduce_bf16(const void *mc)
-{ return emu_mc_reduce<__nv_bfloat16>(mc, [](__nv_bfloat16 a, __nv_bfloat16 b) { return __float2bfloat16_rn(__bfloat162float(a) + __bfloat162float(b)); }); }
+{ return emu_mc_reduce_acc_f32<__nv_bfloat16>(mc, [](__nv_bfloat16 x) { return __bfloat162float(x); }, [](float x) { return __float2bfloat16_rn(x); }); }
 static inline uint4 mc_ld_reduce_f16(const void *mc)
-{ return emu_mc_reduce<__half>(mc, [](__half a, __half b) { return __float2half_rn(__half2float(a) + __half2float(b)); }); }
+{ return emu_mc_reduce_acc_f32<__half>(mc, [](__half x) { return __half2float(x); }, [](float x) { return __float2half_rn(x); }); }
 #define NVL_EMU_RED(_name, _E, _expr) static inline uint4 _name(const void *mc) { return emu_mc_reduce<_E>(mc, [](_E a, _E b) { return (_E)(_expr); }); }
 NVL_EMU_RED(mc_red_add_s32, int32_t, a + b) NVL_EMU_RED(mc_red_add_u32, uint32_t, a + b) NVL_EMU_RED(mc_red_min_s32, int32_t, a < b ? a : b) NVL_EMU_RED(mc_red_max_s32, int32_t, a > b ? a : b)
 NVL_EMU_RED(mc_red_min_u32, uint32_t, a < b ? a : b) NVL_EMU_RED(mc_red_max_u32, uint32_t, a > b ? a : b) NVL_EMU_RED(mc_red_and_b32, uint32_t, a & b) NVL_EMU_RED(mc_red_or_b32, uint32_t, a | b)

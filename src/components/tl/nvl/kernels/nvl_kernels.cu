@@ -211,12 +211,9 @@ __global__ void __launch_bounds__(NVL_THREADS_MAX, 2) nvl_exchange_kernel(nvl_xc
 /* ------------------------------------------------------------------ */
 /* host-side launchers                                                 */
 /* ------------------------------------------------------------------ */
-#ifndef NVL_HOST_EMU /* tests/emu includes the kernels above and calls them directly */
-extern "C" size_t nvl_dt_size(int dt)
-{
-    static const size_t s[NVL_DT_LAST] = {1, 2, 4, 8, 1, 2, 4, 8, 2, 4, 8, 2, 8, 16};
-    return dt >= 0 && dt < NVL_DT_LAST ? s[dt] : 0;
-}
+/* the datatype / operator tables are also compiled into the host emulation that checks every supported pair
+ * (tests/emu/nvl_emu_numerics.cpp defines NVL_EMU_SUPPORT_TABLES) */
+#if !defined(NVL_HOST_EMU) || defined(NVL_EMU_SUPPORT_TABLES)
 extern "C" int nvl_dt_supports_op(int dt, int op)
 {
     if (dt < 0 || dt >= NVL_DT_LAST || op < 0 || op >= NVL_OP_LAST) return 0;
@@ -232,6 +229,14 @@ extern "C" int nvl_nvls_supports(int dt, int op)
     if (dt == NVL_DT_I32 || dt == NVL_DT_U32 || dt == NVL_DT_I64 || dt == NVL_DT_U64)
         return op == NVL_OP_SUM || op == NVL_OP_MIN || op == NVL_OP_MAX || op == NVL_OP_BAND || op == NVL_OP_BOR || op == NVL_OP_BXOR;
     return 0;
+}
+#endif
+
+#ifndef NVL_HOST_EMU /* tests/emu includes the kernels above and calls them directly */
+extern "C" size_t nvl_dt_size(int dt)
+{
+    static const size_t s[NVL_DT_LAST] = {1, 2, 4, 8, 1, 2, 4, 8, 2, 4, 8, 2, 8, 16};
+    return dt >= 0 && dt < NVL_DT_LAST ? s[dt] : 0;
 }
 
 typedef cudaError_t (*nvl_red_launch_fn)(const nvl_red_args_t *, int, int, cudaStream_t);

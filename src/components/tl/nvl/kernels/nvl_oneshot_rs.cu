@@ -19,7 +19,6 @@ static __device__ __forceinline__ void oneshot_rs_body(const nvl_red_args_t &a, 
     const T *src = static_cast<const T *>(a.src);
     T *dst = static_cast<T *>(a.dst);
     const size_t slot = (size_t)((seq & 1) * NVL_MAX_PEERS) * NVL_LL_MAX;
-    const float inv_n = 1.0f / (float)N;
 
     /* push: block p of my vector -> slot `me` of member p; CTA b handles the same vector range of a block on both sides */
     for (int i = 1; i < N; i++) {
@@ -54,7 +53,7 @@ static __device__ __forceinline__ void oneshot_rs_body(const nvl_red_args_t &a, 
             VecAcc<T, OP> acc; acc.set(x[0]);
 #pragma unroll
             for (int i = 1; i < NVL_MAX_PEERS; i++) if (i < N) acc.add(x[i]);
-            store_dst_vec<T>(dst, v * E, cnt, dal, acc.get(inv_n, N));
+            store_dst_vec<T>(dst, v * E, cnt, dal, acc.get(N));
         }
     }
 }

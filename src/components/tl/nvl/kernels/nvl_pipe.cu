@@ -89,7 +89,6 @@ template <typename T, int OP> static __device__ __forceinline__ void pipe_reduce
     constexpr int E = 16 / sizeof(T);
     constexpr int U = NVL_BW_U;
     const int me = a.team.rank;
-    const float inv_n = 1.0f / (float)a.team.size;
     size_t e0, j0, j1; chunk_range<T>(pl, g, k, e0, j0, j1);
     const size_t rc = slice_cnt(a, pl, me) > e0 ? dmin(g.cap_e, slice_cnt(a, pl, me) - e0) : 0;
     const size_t jend = dmin(j1, (rc + E - 1) / E);
@@ -103,13 +102,13 @@ template <typename T, int OP> static __device__ __forceinline__ void pipe_reduce
 #pragma unroll
         for (int u = 0; u < U; u++) {
             uint4 v = r[u];
-            if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(inv_n, a.team.size); }
+            if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(a.team.size); }
             mc_st_v4(mc + (j + (size_t)u * rnt) * 16, v); /* the padding lanes of a ragged last vector are reduced and stored too: they stay inside the slot */
         }
     }
     for (; j < jend; j += rnt) {
         uint4 v = McRed<T, OP>::ld(mc + j * 16);
-        if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(inv_n, a.team.size); }
+        if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(a.team.size); }
         mc_st_v4(mc + j * 16, v);
     }
 }

@@ -83,7 +83,6 @@ static __device__ __forceinline__ void oneshot_body(const nvl_red_args_t &a, nvl
     const size_t per = (nvec + gridDim.x - 1) / gridDim.x, v0 = dmin((size_t)blockIdx.x * per, nvec), v1 = dmin(v0 + per, nvec);
     const bool sal = ((uintptr_t)src & 15) == 0, dal = ((uintptr_t)dst & 15) == 0;
     const size_t slot = (size_t)((seq & 1) * NVL_MAX_PEERS) * NVL_LL_MAX;
-    const float inv_n = 1.0f / (float)N;
 
     for (size_t v = v0 + threadIdx.x; v < v1; v += blockDim.x) {
         uint4 x = load_src_vec<T>(src, v * E, n, sal);
@@ -100,16 +99,20 @@ static __device__ __forceinline__ void oneshot_body(const nvl_red_args_t &a, nvl
         bs.spin(t, &mine->ll_flags[blockIdx.x][threadIdx.x], seq);
     }
     __syncthreads();
+    /* reduce in rank order 0..N-1 on every rank (vector p: my own source for p == me, slot p of my heap otherwise), so that
+     * every rank stores the same bits - floating-point addition is not associative, and replicas of a data-parallel model
+     * drift apart when their gradients differ in the last bit.  The reads hit my own heap, so their order costs nothing.
+     * x[] is only indexed with unrolled constants: no local-memory stack. */
     const char *mybase = t.heap[me] + NVL_LL_OFFSET + slot;
     for (size_t v = v0 + threadIdx.x; v < v1; v += blockDim.x) {
         uint4 x[NVL_MAX_PEERS];
-        x[0] = load_src_vec<T>(src, v * E, n, sal);
 #pragma unroll
-        for (int i = 1; i < NVL_MAX_PEERS; i++) if (i < N) { int p = me + i; if (p >= N) p -= N; x[i] = ld_peer_v4(mybase + (size_t)p * NVL_LL_MAX + v * 16); }
+        for (int p = 0; p < NVL_MAX_PEERS; p++)
+            if (p < N) x[p] = p == me ? load_src_vec<T>(src, v * E, n, sal) : ld_peer_v4(mybase + (size_t)p * NVL_LL_MAX + v * 16);
         VecAcc<T, OP> acc; acc.set(x[0]);
 #pragma unroll
-        for (int i = 1; i < NVL_MAX_PEERS; i++) if (i < N) acc.add(x[i]);
-        store_dst_vec<T>(dst, v * E, n, dal, acc.get(inv_n, N));
+        for (int p = 1; p < NVL_MAX_PEERS; p++) if (p < N) acc.add(x[p]);
+        store_dst_vec<T>(dst, v * E, n, dal, acc.get(N));
     }
 }
 
@@ -191,7 +194,7 @@ template <typename T> static __device__ __forceinline__ void make_plan(const nvl
  * 2 x 512 threads per SM).  CN = team size when it is one of the common ones (2, 4, 8): every bound below is then a
  * compile-time constant and the loop carries no predicates; CN = 0 is the generic team size. */
 template <typename T, int OP, int CN, int NP, int U, typename SRC, typename ST>
-static __device__ __forceinline__ void reduce_core(int n_rt, size_t j0, size_t jend, float inv_n, SRC src_of, ST store)
+static __device__ __forceinline__ void reduce_core(int n_rt, size_t j0, size_t jend, SRC src_of, ST store)
 {
     const int N = CN ? CN : n_rt;
     const size_t nt = blockDim.x;
@@ -238,7 +241,7 @@ static __device__ __forceinline__ void reduce_core(int n_rt, size_t j0, size_t j
 #pragma unroll
         for (int u = 0; u < U; u++) {
             const size_t jj = j + u * nt;
-            if (jj < jend) store(jj, acc[u].get(inv_n, N));
+            if (jj < jend) store(jj, acc[u].get(N));
         }
     }
 }
@@ -249,7 +252,7 @@ template <int CN> struct RedShape { static constexpr int NP = CN == 2 ? 2 : 4, U
 /* phase B of the staged kernel over P2P: sources = the members' staging areas, result -> every member's staging area
  * (allreduce), the root's (reduce) or straight into my destination block (reduce_scatter) */
 template <typename T, int OP, int CN>
-static __device__ __forceinline__ void reduce_p2p(const nvl_red_args_t &a, size_t base, size_t j0, size_t jend, T *db, size_t rc, bool dal, float inv_n)
+static __device__ __forceinline__ void reduce_p2p(const nvl_red_args_t &a, size_t base, size_t j0, size_t jend, T *db, size_t rc, bool dal)
 {
     constexpr int E = 16 / sizeof(T);
     const int N = CN ? CN : a.team.size, me = a.team.rank;
@@ -261,11 +264,11 @@ static __device__ __forceinline__ void reduce_p2p(const nvl_red_args_t &a, size_
         } else if (a.kind == NVL_RED_REDUCE) st_v4(data_of(a.team, a.root) + base + jj * 16, r);
         else store_dst_vec<T>(db, jj * E, rc, dal, r);
     };
-    reduce_core<T, OP, CN, RedShape<CN>::NP, RedShape<CN>::U>(N, j0, jend, inv_n, src_of, store);
+    reduce_core<T, OP, CN, RedShape<CN>::NP, RedShape<CN>::U>(N, j0, jend, src_of, store);
 }
 
 template <typename T, int OP, int U>
-static __device__ __forceinline__ void reduce_nvls(const nvl_red_args_t &a, size_t base, size_t j0, size_t jend, T *db, size_t rc, bool dal, float inv_n)
+static __device__ __forceinline__ void reduce_nvls(const nvl_red_args_t &a, size_t base, size_t j0, size_t jend, T *db, size_t rc, bool dal)
 {
     constexpr int E = 16 / sizeof(T);
     const size_t nt = blockDim.x;
@@ -279,7 +282,7 @@ static __device__ __forceinline__ void reduce_nvls(const nvl_red_args_t &a, size
             const size_t jj = j + u * nt;
             if (jj < jend) {
                 uint4 v = r[u];
-                if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(inv_n, a.team.size); }
+                if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(a.team.size); }
                 if (a.kind == NVL_RED_ALLREDUCE) mc_st_v4(mc + jj * 16, v);
                 else if (a.kind == NVL_RED_REDUCE) st_v4(data_of(a.team, a.root) + base + jj * 16, v);
                 else store_dst_vec<T>(db, jj * E, rc, dal, v);
@@ -298,7 +301,6 @@ static __device__ __forceinline__ void staged_body(const nvl_red_args_t &a, Bloc
     const T *src = static_cast<const T *>(a.src);
     T *dst = static_cast<T *>(a.dst);
     const size_t cap_bytes = pl.cap_e * sizeof(T);
-    const float inv_n = 1.0f / (float)N;
     char *mydata = data_of(t, me);
 
     for (int k = 0; k < pl.rounds; k++) {
@@ -334,8 +336,8 @@ static __device__ __forceinline__ void staged_body(const nvl_red_args_t &a, Bloc
             const size_t jend = dmin(j1, (rc + E - 1) / E), base = (size_t)me * cap_bytes;
             T *db = dst + (a.kind == NVL_RED_REDUCE_SCATTER ? 0 : slice_off(a, pl, me)) + e0;
             const bool dal = ((uintptr_t)db & 15) == 0;
-            if constexpr (MODE < 0) reduce_nvls<T, OP, NVL_BW_U>(a, base, j0, jend, db, rc, dal, inv_n);
-            else reduce_p2p<T, OP, MODE>(a, base, j0, jend, db, rc, dal, inv_n);
+            if constexpr (MODE < 0) reduce_nvls<T, OP, NVL_BW_U>(a, base, j0, jend, db, rc, dal);
+            else reduce_p2p<T, OP, MODE>(a, base, j0, jend, db, rc, dal);
         }
         bs.barrier(t, 2 * k + 2);
 
@@ -394,7 +396,7 @@ template <typename T> static cudaError_t nvl_reduce_staged_kernel_launch(const n
  * neighbour (i = 0: myself).  Inside the unrolled loops every index is a compile-time constant, so the addresses are formed
  * straight from the constant bank that holds the kernel parameters - no pointer table in registers, nothing on the stack. */
 template <typename T, int OP, int CN>
-static __device__ __forceinline__ void direct_p2p(const nvl_red_args_t &a, size_t so, size_t j0, size_t jend, float inv_n)
+static __device__ __forceinline__ void direct_p2p(const nvl_red_args_t &a, size_t so, size_t j0, size_t jend)
 {
     const int N = CN ? CN : a.team.size;
     const int rooti = a.kind == NVL_RED_REDUCE ? (a.root - a.team.rank + N) % N : 0;
@@ -406,7 +408,7 @@ static __device__ __forceinline__ void direct_p2p(const nvl_red_args_t &a, size_
             for (int i = 0; i < N; i++) st_v4(a.d.dst[i] + so + jj * 16, r);
         } else st_v4(single + jj * 16, r);
     };
-    reduce_core<T, OP, CN, RedShape<CN>::NP, RedShape<CN>::U>(N, j0, jend, inv_n, src_of, store);
+    reduce_core<T, OP, CN, RedShape<CN>::NP, RedShape<CN>::U>(N, j0, jend, src_of, store);
 }
 
 template <typename T, int OP, int CN>
@@ -419,17 +421,16 @@ static __device__ __forceinline__ void direct_body(const nvl_red_args_t &a, cons
     const size_t cnt = slice_cnt(a, pl, me), nfull = cnt / E, per = (nfull + nb - 1) / nb;
     const size_t j0 = dmin((size_t)b * per, nfull), j1 = dmin(j0 + per, nfull);
     const size_t so = slice_off(a, pl, me) * sizeof(T);
-    const float inv_n = 1.0f / (float)N;
     /* in flight per thread: U x NP 16-byte loads; 2 CTAs x 512 threads per SM keep > 64 KB outstanding per SM, far above
      * the NVLink bandwidth-delay product */
-    direct_p2p<T, OP, CN>(a, so, j0, j1, inv_n); /* the team size class is a kernel template parameter: each class gets its own register allocation */
+    direct_p2p<T, OP, CN>(a, so, j0, j1); /* the team size class is a kernel template parameter: each class gets its own register allocation */
     /* ragged tail of the slice (fewer than E elements): one thread, element by element (cold; dynamic constant-bank indexing) */
     if (b == nb - 1 && threadIdx.x == 0 && nfull * E < cnt) {
         const int rooti = a.kind == NVL_RED_REDUCE ? (a.root - me + N) % N : 0;
         for (size_t e = nfull * E; e < cnt; e++) {
             A acc = to_acc<T>(reinterpret_cast<const T *>(a.d.src[0] + so)[e]);
             for (int i = 1; i < N; i++) acc = OpFn<OP, A>::f(acc, to_acc<T>(reinterpret_cast<const T *>(a.d.src[i] + so)[e]));
-            acc = avg_scale<OP, A>(acc, inv_n, N);
+            acc = avg_scale<OP, A>(acc, N);
             if (a.kind == NVL_RED_ALLREDUCE) { for (int i = 0; i < N; i++) reinterpret_cast<T *>(a.d.dst[i] + so)[e] = from_acc<T>(acc); }
             else if (a.kind == NVL_RED_REDUCE) reinterpret_cast<T *>(a.d.dst[rooti] + so)[e] = from_acc<T>(acc);
             else static_cast<T *>(a.dst)[e] = from_acc<T>(acc); /* reduce_scatter(v): my block, already a local pointer */
@@ -501,7 +502,7 @@ template <typename T> static cudaError_t nvl_reduce_direct_kernel_launch(const n
 /* ------------------------------------------------------------------ */
 /* acc[j] = op(peer[j], mine[j]) for my block's vectors of one slice; optionally scaled (AVG) and mirrored into dst */
 template <typename T, int OP>
-static __device__ __forceinline__ void step_reduce(const char *peer, char *mine, size_t j0, size_t jend, bool last, float inv_n, int N, T *db, size_t rc, bool dal)
+static __device__ __forceinline__ void step_reduce(const char *peer, char *mine, size_t j0, size_t jend, bool last, int N, T *db, size_t rc, bool dal)
 {
     constexpr int E = 16 / sizeof(T);
     const size_t nt = blockDim.x;
@@ -512,7 +513,7 @@ static __device__ __forceinline__ void step_reduce(const char *peer, char *mine,
 #pragma unroll
         for (int u = 0; u < 4; u++) if (j + u * nt < jend) {
             VecAcc<T, OP> acc; acc.set(y[u]); acc.add(x[u]);
-            const uint4 r = acc.get(last ? inv_n : 1.0f, last ? N : 1); /* get() scales for AVG only; partial sums must stay unscaled */
+            const uint4 r = acc.get(last ? N : 1); /* get() scales for AVG only; partial sums must stay unscaled */
             st_v4(mine + (j + u * nt) * 16, r);
             if (db) store_dst_vec<T>(db, (j + u * nt) * E, rc, dal, r);
         }
@@ -545,7 +546,6 @@ static __device__ __forceinline__ void steps_body(const nvl_red_args_t &a, Block
     const T *src = static_cast<const T *>(a.src);
     T *dst = static_cast<T *>(a.dst);
     const size_t cap_bytes = pl.cap_e * sizeof(T);
-    const float inv_n = 1.0f / (float)N;
     const size_t nvmax = (pl.slice_max + E - 1) / E, per = (nvmax + nb - 1) / nb;
     const size_t j0 = dmin((size_t)b * per, nvmax), j1 = dmin(j0 + per, nvmax);
     char *mydata = data_of(t, me);
@@ -573,7 +573,7 @@ static __device__ __forceinline__ void steps_body(const nvl_red_args_t &a, Block
             const int c = (me - 2 - s + 3 * N) % N;
             const bool last = s + 2 == N;
             T *db = last ? SLICE_DST(c) : nullptr; /* c == me in the last step */
-            step_reduce<T, OP>(left + (size_t)c * cap_bytes, mydata + (size_t)c * cap_bytes, j0, SLICE_JEND(c), last, inv_n, N, db, slice_cnt(a, pl, c), db && ((uintptr_t)db & 15) == 0);
+            step_reduce<T, OP>(left + (size_t)c * cap_bytes, mydata + (size_t)c * cap_bytes, j0, SLICE_JEND(c), last, N, db, slice_cnt(a, pl, c), db && ((uintptr_t)db & 15) == 0);
             bs.barrier(t, ++phase);
         }
         if (allred) for (int s = 0; s + 1 < N; s++) {
@@ -592,7 +592,7 @@ static __device__ __forceinline__ void steps_body(const nvl_red_args_t &a, Block
             char *pd = data_of(t, partner);
             for (int c = klo; c < khi; c++) {
                 T *db = last ? SLICE_DST(c) : nullptr;
-                step_reduce<T, OP>(pd + (size_t)c * cap_bytes, mydata + (size_t)c * cap_bytes, j0, SLICE_JEND(c), last, inv_n, N, db, slice_cnt(a, pl, c), db && ((uintptr_t)db & 15) == 0);
+                step_reduce<T, OP>(pd + (size_t)c * cap_bytes, mydata + (size_t)c * cap_bytes, j0, SLICE_JEND(c), last, N, db, slice_cnt(a, pl, c), db && ((uintptr_t)db & 15) == 0);
             }
             lo = klo; hi = khi;
             bs.barrier(t, ++phase);

@@ -24,7 +24,6 @@ static __device__ __forceinline__ void symm_body(const nvl_red_args_t &a, BlockS
     const int N = t.size, me = t.rank;
     const bool rs = a.kind == NVL_RED_REDUCE_SCATTER;   /* reduce_scatter(v): only src is symmetric, my block goes to the local a.dst */
     const size_t so = (size_t)(a.d.src[0] - t.heap[me]), dof = rs ? 0 : (size_t)(a.d.dst[0] - t.heap[me]);
-    const float inv_n = 1.0f / (float)N;
     const size_t nt = blockDim.x;
 
     bs.barrier(t, 1);
@@ -42,13 +41,13 @@ static __device__ __forceinline__ void symm_body(const nvl_red_args_t &a, BlockS
 #pragma unroll
             for (int u = 0; u < U; u++) {
                 uint4 v = r[u];
-                if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(inv_n, N); }
+                if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(N); }
                 store_dst_vec<T>(db, (j + (size_t)u * nt) * E, cnt, dal, v);   /* bounds-checked: the ragged last vector is cut at cnt */
             }
         }
         for (; j < j1; j += nt) {
             uint4 v = McRed<T, OP>::ld(mcs + j * 16);
-            if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(inv_n, N); }
+            if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(N); }
             store_dst_vec<T>(db, j * E, cnt, dal, v);
         }
     } else {
@@ -65,13 +64,13 @@ static __device__ __forceinline__ void symm_body(const nvl_red_args_t &a, BlockS
 #pragma unroll
             for (int u = 0; u < U; u++) {
                 uint4 v = r[u];
-                if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(inv_n, N); }
+                if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(N); }
                 mc_st_v4(mcd + (j + (size_t)u * nt) * 16, v);
             }
         }
         for (; j < jfull; j += nt) {
             uint4 v = McRed<T, OP>::ld(mcs + j * 16);
-            if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(inv_n, N); }
+            if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(N); }
             mc_st_v4(mcd + j * 16, v);
         }
         /* ragged end of the vector (only the last non-empty slice can have one): the 16-byte load stays inside the 256-byte
@@ -79,7 +78,7 @@ static __device__ __forceinline__ void symm_body(const nvl_red_args_t &a, BlockS
          * member's unicast mapping instead */
         if (nfull < nv && nfull >= j0 && nfull < j1 && threadIdx.x == 0) {
             uint4 v = McRed<T, OP>::ld(mcs + nfull * 16);
-            if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(inv_n, N); }
+            if (OP == NVL_OP_AVG) { VecAcc<T, OP> acc; acc.set(v); v = acc.get(N); }
             for (int p = 0; p < N; p++)
                 store_dst_vec<T>(reinterpret_cast<T *>(t.heap[p] + dof) + slice_off(a, pl, me), nfull * E, cnt, false, v);
         }
